@@ -92,6 +92,42 @@ def full_compare(a, b):
     return bad
 
 
+DUMP_WINDOWS, DUMP_SEGMENTS, DUMP_BASES = 1 << 15, 1 << 16, 1 << 20      # sample sizes of --dump-outputs: at most about 45 MB of .npy files
+
+
+def dump_outputs(path, win_out, reads_out):
+    """--dump-outputs: what a caller of the timed paths receives, as DIR/<name>.npy in float32 / float64, so that two builds can be compared
+    output for output.  win_out = (res, cons, ops) of the last step of the device-resident leg: the result records of a fixed sample of windows,
+    with the consensus bytes and placement trace a window has (status 1: the first clen / nops bytes; zeros elsewhere, as those bytes are
+    undefined).  reads_out = (seg, chars) of the last e2e step, or None when that leg did not run: the segment records and the corrected bases,
+    both sampled when larger than the sample.  Each sample is a seeded function of the array's length alone."""
+    rng = np.random.default_rng(20240601)
+
+    def sample(n, k):
+        return np.arange(n) if n <= k else np.unique(rng.integers(0, n, k))
+    res, cons, ops = win_out
+    n = len(res)
+    wi = sample(n, DUMP_WINDOWS)
+    r = res[wi]
+    ok = r["status"] == 1
+    c = np.asarray(cons).reshape(n, 64)[wi]
+    o = np.asarray(ops).reshape(n, 128)[wi]
+    arrays = {"window_index": wi.astype(np.float64),
+              "window_consensus": np.where(ok[:, None] & (np.arange(64)[None, :] < r["clen"][:, None]), c, 0).astype(np.float32),
+              "window_placement": np.where(ok[:, None] & (np.arange(128)[None, :] < r["nops"][:, None]), o, 0).astype(np.float32)}
+    arrays.update(("window_" + f, r[f].astype(np.float64)) for f in res.dtype.names)
+    if reads_out is not None:
+        seg, chars = reads_out
+        si, bi = sample(len(seg), DUMP_SEGMENTS), sample(len(chars), DUMP_BASES)
+        arrays["read_segment_index"] = si.astype(np.float64)
+        arrays.update(("read_segment_" + f, seg[si][f].astype(np.float64)) for f in seg.dtype.names)
+        arrays["read_base_index"] = bi.astype(np.float64)
+        arrays["read_bases"] = chars[bi].astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def effective_cpus():
     """CPUs this process may really use: affinity mask and cgroup quota (os.cpu_count() ignores both)"""
     n = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
@@ -182,7 +218,13 @@ def main():
     ap.add_argument("--truth-reads", type=int, default=400, help="corrected reads compared with the simulated truth (0 = off)")
     ap.add_argument("--cli", type=int, default=1, help="N=1 only: also time the `daccord` binary on the same data as .las / .db files (wall clock of the whole process)")
     ap.add_argument("--cli-oracle-reads", type=int, default=24, help="A-reads on which the oracle's file driver (all threads) is run beside the binary for a byte comparison of the FastA (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (window results of a fixed sample of windows, corrected reads) as DIR/<name>.npy, rank 0's shard")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times a sample whose size depends on the host's speed, so it has no fixed outputs to write")
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -319,7 +361,7 @@ def main():
         pile_wall = time.perf_counter() - t0
         pile_same = not full_compare((res_ref, cons_ref, ops_ref), out).any()
     # ---- e2e: the whole read-level path on the GPU: overlaps in, corrected bases out (dcu_pile + launch + dcu_vote); D2H = corrected bases only
-    full_wall, full_same, full_d2h, truth, e2e_parts = None, None, 0, None, None
+    full_wall, full_same, full_d2h, truth, e2e_parts, reads_out = None, None, 0, None, None, None
     if gpu_pile:
         eng.pile(ovl, trace, ds.tspace, boff, rlen, advance=args.a, maxalign=maxalign); eng.launch(); seg, chars = eng.vote()      # warm-up
         chars_p = torch.empty(int(len(chars) * 1.02) + 4096, dtype=torch.uint8).pin_memory().numpy()     # pinned target of the corrected bases, like the other host buffers of the step
@@ -339,6 +381,8 @@ def main():
         full_wall = time.perf_counter() - t0
         e2e_parts = {"dcu_pile_ms": 1e3 * tp / args.steps, "dcu_launch_ms": 1e3 * tl / args.steps, "dcu_vote_and_get_corrected_ms": 1e3 * tv / args.steps}
         gfasta = format_segments(seg, chars)[0]
+        if args.dump_outputs:
+            reads_out = (seg.copy(), chars.copy())      # chars lies in chars_p, which the two-in-flight leg below writes again
         full_same = bool(gfasta == fasta)
         full_d2h = int(chars.nbytes + seg.nbytes + 16 * nwin)       # + the window descriptors dcu_vote reads back to lay out the reads
         if keep_truth and rank == 0:
@@ -487,6 +531,8 @@ def main():
                                 "sample": "first %d windows of the step, %.1f s" % (n, t), "gpu_results_identical_on_sample": not diff.any(),
                                 "compared": "result record, consensus bytes and placement trace of every sampled window", "differing_windows": int(diff.sum()),
                                 "note": "CPU restatement of gt1/daccord (bit-parallel scoring, -march=x86-64-v3), not the upstream binary: GPU/CPU ratios are upper bounds vs real daccord"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, (res_ref, cons_ref, ops_ref), reads_out)
     print(json.dumps(line))
     if dist is not None:
         dist.destroy_process_group()

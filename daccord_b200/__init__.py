@@ -153,7 +153,10 @@ class Engine:
         return {"launches": a.value, "hard_windows": b.value, "second_pass_windows": c.value, "lost_windows": d.value, "smem_warps": e.value, "smem_bytes_per_warp": f.value}
 
     def tables(self, which):
+        """table `which` (0 DPn, 1 DPsq, 2 VSq, 3 suplo/suphi pairs, 4 klim, 5 NP/MS/KLIMN) as read back from device memory"""
         n = self.lib.dcu_get_tables(self.ctx, C.c_int(which), None, C.c_int64(0))
+        if n < 0:
+            raise DcuError("dcu_get_tables: " + self.lib.dcu_last_error(self.ctx).decode())
         out = np.zeros(n, np.float64)
         self.lib.dcu_get_tables(self.ctx, C.c_int(which), _p(out), C.c_int64(n))
         return out

@@ -453,6 +453,7 @@ int dcu_create(const dcu_params* p, int device, dcu_ctx** out) {
   if (p->k_lo < 3 || p->k_hi > 14 || p->k_lo > p->k_hi) return DCU_ERR_UNSUPPORTED;
   if (p->max_ff < p->min_ff || p->min_ff < 0) return DCU_ERR_PARAM;
   if (!(p->p_i >= 0 && p->p_i < 1 && p->p_d >= 0 && p->p_d < 1)) return DCU_ERR_PARAM;
+  if (!(p->est_cor >= 0 && p->est_cor <= 1)) return DCU_ERR_PARAM;     // a probability (NaN fails too): the k-mer limits are its binomial quantiles
   dcu_ctx* ctx = new (std::nothrow) dcu_ctx();
   if (!ctx) return DCU_ERR_PARAM;
   ctx->device = device; ctx->prm = *p;
@@ -978,13 +979,23 @@ int dcu_last_stats2(dcu_ctx* ctx, uint64_t* second_pass_windows, uint64_t* lost_
   return DCU_OK;
 }
 
+// the tables as the kernel reads them: copied back from the device buffers, not the host copy they were uploaded from
 int64_t dcu_get_tables(dcu_ctx* ctx, int which, double* out, int64_t cap) {
   if (!ctx) return -1;
-  std::vector<double> v; auto& H = ctx->HT;
-  if (which == 0) v = H.DPn; else if (which == 1) v = H.DPsq;
-  else if (which == 2) { for (int l = 0; l < H.NP; ++l) for (int q = 0; q < H.MS; ++q) v.push_back((double)H.VSq[(size_t)q * H.NP + l]); }
-  else if (which == 3) for (int i = 0; i < H.MS; ++i) { v.push_back(H.suplo[i]); v.push_back(H.suphi[i]); }
-  else if (which == 4) for (auto x : H.klim) v.push_back((double)x);
+  const auto& H = ctx->HT;
+  std::vector<double> DPn(H.DPn.size()), DPsq(H.DPsq.size());
+  std::vector<unsigned long long> VSq(H.VSq.size()), klim(H.klim.size());
+  std::vector<uint16_t> suplo(H.suplo.size()), suphi(H.suphi.size());
+  if (cudaSetDevice(ctx->device) != cudaSuccess) return -1;
+  for (auto c : {cudaMemcpy(DPn.data(), ctx->dDPn.p, DPn.size() * 8, cudaMemcpyDeviceToHost), cudaMemcpy(DPsq.data(), ctx->dDPsq.p, DPsq.size() * 8, cudaMemcpyDeviceToHost),
+                 cudaMemcpy(VSq.data(), ctx->dVSq.p, VSq.size() * 8, cudaMemcpyDeviceToHost), cudaMemcpy(klim.data(), ctx->dklim.p, klim.size() * 8, cudaMemcpyDeviceToHost),
+                 cudaMemcpy(suplo.data(), ctx->dsuplo.p, suplo.size() * 2, cudaMemcpyDeviceToHost), cudaMemcpy(suphi.data(), ctx->dsuphi.p, suphi.size() * 2, cudaMemcpyDeviceToHost)})
+    if (c != cudaSuccess) { ctx->err = std::string("dcu_get_tables: ") + cudaGetErrorString(c); return -1; }
+  std::vector<double> v;
+  if (which == 0) v = DPn; else if (which == 1) v = DPsq;
+  else if (which == 2) { for (int l = 0; l < H.NP; ++l) for (int q = 0; q < H.MS; ++q) v.push_back((double)VSq[(size_t)q * H.NP + l]); }
+  else if (which == 3) for (int i = 0; i < H.MS; ++i) { v.push_back(suplo[i]); v.push_back(suphi[i]); }
+  else if (which == 4) for (auto x : klim) v.push_back((double)x);
   else if (which == 5) { v.push_back(H.NP); v.push_back(H.MS); v.push_back(H.KLIMN); }
   if (out && (int64_t)v.size() <= cap) memcpy(out, v.data(), v.size() * sizeof(double));
   return (int64_t)v.size();

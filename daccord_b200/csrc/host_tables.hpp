@@ -21,6 +21,29 @@ struct HostTables {
   std::vector<unsigned long long> klim;          // [nk][KLIMN]
 };
 
+// Smallest m with Binomial(n, p) CDF(m) >= lim, n if none.  The pmf is walked unnormalised from its mode (term 1) outward by the
+// ratio recurrence, so no term underflows for any n (q^n, the usual starting term, is 0 or a denormal once n ln q < -708 and
+// then wrecks the limit of deep windows).  A walk stops after its first term below 1e-30: the terms fall monotonically away from
+// the mode, so what is dropped is below n * 1e-30 of a total >= 1.  The CDF is the running sum in ascending m against the walk's
+// own total.  Same operations in the same order as oracle/tables.hpp binomRowUpperLimit.
+inline unsigned long long binom_upper_limit(double p, unsigned long long n, double lim) {
+  double q = 1.0 - p;
+  if (!(q > 0.0)) return n;                                 // p = 1 (and NaN)
+  const double up = p / q, down = q / p;
+  const double mf = std::floor((double)(n + 1) * p);
+  const unsigned long long M = mf <= 0.0 ? 0 : (mf >= (double)n ? n : (unsigned long long)mf);
+  std::vector<double> hi(1, 1.0), lo;                       // hi[i]: term of m = M + i; lo[i]: term of m = M - 1 - i
+  for (unsigned long long m = M; m < n && hi.back() >= 1e-30; ++m) hi.push_back(hi.back() * (double)(n - m) / (double)(m + 1) * up);
+  for (unsigned long long m = M; m > 0 && (lo.empty() || lo.back() >= 1e-30); --m) lo.push_back((lo.empty() ? 1.0 : lo.back()) * (double)m / (double)(n - m + 1) * down);
+  double total = 0.0;
+  for (size_t i = lo.size(); i-- > 0;) total += lo[i];
+  for (double t : hi) total += t;
+  double sum = 0.0;
+  for (size_t i = lo.size(); i-- > 0;) { sum += lo[i]; if (sum >= lim * total) return M - 1 - i; }
+  for (size_t i = 0; i < hi.size(); ++i) { sum += hi[i]; if (sum >= lim * total) return M + i; }
+  return n;
+}
+
 // P(read offset = j | true offset = l): (l+1)-fold geometric insertion law convolved with Binomial(l,p_d) deletions
 inline void build_tables(int w, double p_i, double p_d, double est_cor, int k_lo, int k_hi, int klimn, HostTables& T) {
   const int NP = w + 1;
@@ -112,20 +135,8 @@ inline void build_tables(int w, double p_i, double p_d, double est_cor, int k_lo
   T.klim.assign((size_t)T.nk * klimn, 0ull);
   for (int kk = k_lo; kk <= k_hi; ++kk) {
     double pk = std::pow(est_cor, (double)kk);
-    for (int n = 0; n < klimn; ++n) {
-      unsigned long long lim = (unsigned long long)n;
-      if (pk == 0.0) lim = 0;
-      else {
-        double q = 1.0 - pk;
-        if (q != 0.0) {
-          double term = 1.0;
-          for (int t = 0; t < n; ++t) term *= q;
-          double ratio = pk / q, sum = 0.0;
-          for (int m = 0; m <= n; ++m) { sum += term; if (sum >= 0.99) { lim = (unsigned long long)m; break; } term = term * (double)(n - m) / (double)(m + 1) * ratio; }
-        }
-      }
-      T.klim[(size_t)(kk - k_lo) * klimn + n] = lim;
-    }
+    for (int n = 0; n < klimn; ++n)
+      T.klim[(size_t)(kk - k_lo) * klimn + n] = pk == 0.0 ? 0ull : binom_upper_limit(pk, (unsigned long long)n, 0.99);
   }
 }
 

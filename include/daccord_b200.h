@@ -126,7 +126,7 @@ int dcu_last_stats(dcu_ctx* ctx, uint64_t* launches, uint64_t* hard_windows);
  * (status DCU_WIN_OVERFLOW), warps per SM and shared-memory bytes per warp of a first pass that keeps data in shared memory (the hybrid
  * pass: k-mer table only, 32 warps; DCU_SMEM=1: the graph, 12-16 warps; 0 warps = plain HBM first pass) */
 int dcu_last_stats2(dcu_ctx* ctx, uint64_t* second_pass_windows, uint64_t* lost_windows, uint32_t* smem_warps, uint32_t* smem_bytes_per_warp);
-/* dump the host-built tables (for tests): returns number of doubles written / needed */
+/* dump the tables as they sit in device memory (for tests): returns number of doubles written / needed, -1 on a CUDA error */
 int64_t dcu_get_tables(dcu_ctx* ctx, int which, double* out, int64_t cap);
 const char* dcu_strerror(int code);
 const char* dcu_last_error(dcu_ctx* ctx);

@@ -128,18 +128,25 @@ inline OffsetLikely computeOffsetLikely(uint64_t maxl, double p_i, double p_d) {
   return OL;
 }
 
-// C3
+// C3.  The pmf is walked unnormalised from its mode (term 1) outward by the ratio recurrence, so no term underflows for any n
+// (q^n, the usual starting term, is 0 or a denormal once n ln q < -708).  A walk stops after its first term below 1e-30: the
+// terms fall monotonically away from the mode, so what is dropped is below n * 1e-30 of a total >= 1.  The CDF is the running
+// sum in ascending m against the walk's own total.
 inline uint64_t binomRowUpperLimit(double p, uint64_t n, double lim) {
   double q = 1.0 - p;
-  if (q == 0.0) return n;
-  double term = 1.0;
-  for (uint64_t t = 0; t < n; ++t) term *= q;
-  double ratio = p / q, sum = 0.0;
-  for (uint64_t m = 0; m <= n; ++m) {
-    sum += term;
-    if (sum >= lim) return m;
-    term = term * (double)(n - m) / (double)(m + 1) * ratio;
-  }
+  if (!(q > 0.0)) return n;                                 // p = 1 (and NaN)
+  const double up = p / q, down = q / p;
+  const double mf = std::floor((double)(n + 1) * p);
+  const uint64_t M = mf <= 0.0 ? 0 : (mf >= (double)n ? n : (uint64_t)mf);
+  std::vector<double> hi(1, 1.0), lo;                       // hi[i]: term of m = M + i; lo[i]: term of m = M - 1 - i
+  for (uint64_t m = M; m < n && hi.back() >= 1e-30; ++m) hi.push_back(hi.back() * (double)(n - m) / (double)(m + 1) * up);
+  for (uint64_t m = M; m > 0 && (lo.empty() || lo.back() >= 1e-30); --m) lo.push_back((lo.empty() ? 1.0 : lo.back()) * (double)m / (double)(n - m + 1) * down);
+  double total = 0.0;
+  for (size_t i = lo.size(); i-- > 0;) total += lo[i];
+  for (double t : hi) total += t;
+  double sum = 0.0;
+  for (size_t i = lo.size(); i-- > 0;) { sum += lo[i]; if (sum >= lim * total) return M - 1 - i; }
+  for (size_t i = 0; i < hi.size(); ++i) { sum += hi[i]; if (sum >= lim * total) return M + i; }
   return n;
 }
 
